@@ -3,6 +3,11 @@
 
   python bench.py --gpus N --steps K --warmup W            # B200 engine (torchrun launches one rank per GPU)
   python bench.py --impl reference --steps K --warmup W    # CPU baseline arm (oracle port of the reference, host cores)
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's images (DIR/images.npy)
+
+The inputs are the same on every run. The outputs are not bit-identical from run to run: graph mode times its GEMM
+tile / split-K candidates per process and GroupNorm partial sums meet in fp64 atomics, so two runs of one build differ
+by 1 (of 255) in a few percent of the pixels (5 % on a B200); compare dumps of two builds with that tolerance.
 
 A "step" is one pass of the hot path over one batch: CLIP text encode of [uncond; prompts] -> 51 guided UNet
 evaluations (PLMS-50) -> AutoencoderKL decode -> uint8 images. Weights are seeded random-init of the SD-v1
@@ -28,6 +33,22 @@ METRIC = "images_per_sec_sdv1_512x512_plms50_cfg7.5"
 UNET_GF_PER_SAMPLE = 803.27     # SURVEY.md §8(d): algorithmic GFLOP per UNet evaluation per sample @ 64x64 latent
 VAE_DEC_GF = 2514.5             # per image @ 512x512
 CLIP_GF_PER_PROMPT = 13.0
+DUMP_BYTES = 64 * 10**6         # --dump-outputs writes at most this much in all
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32. An array over its share of DUMP_BYTES is replaced by a fixed,
+    seeded sample of its elements (the same indices for the same shape), so runs of two builds compare element for
+    element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays) // 4 - 32    # float32 elements per array; 128 bytes left for the .npy header
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if a.numel() > budget:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:budget].sort().values
+            a = a.flatten()[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def gemm_dram_traffic():
@@ -233,17 +254,18 @@ def run_gpu(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """Runs `steps` steps between two events; returns (ms, what the last step returned)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms)
+        return float(ms), out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -253,13 +275,16 @@ def run_gpu(args):
     n0 = ops.launch_count()
     if os.environ.get("SDB_PROFILE_RANGE"):   # ncu --profile-from-start off: only the timed steps are captured
         torch.cuda.profiler.start()
-    ms_total = timed(step_resident, args.steps)
+    ms_total, last_img = timed(step_resident, args.steps)
     if os.environ.get("SDB_PROFILE_RANGE"):
         torch.cuda.profiler.stop()
     launches = (ops.launch_count() - n0) // args.steps
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the images the last timed step handed its caller (all ranks' on rank 0), before later steps reuse `gathered`
+        dump_outputs(args.dump_outputs, {"images": torch.cat(gathered) if world > 1 else last_img})
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     # sanity of what was timed (outside the timed region): the latent the 51 evaluations produce is finite and the
     # decoded image is not constant — a NaN anywhere in the UNet would show here
     lat = pipe(ids_d, un_d, x_T=xT_d, return_latent=True)
@@ -395,7 +420,13 @@ def main():
     ap.add_argument("--impl", default="sdb200", choices=["sdb200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--extra-batch", type=int, default=8, help="also time one step at this per-GPU batch (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the uint8 images of the last one as float32 to DIR/images.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "sdb200":
+        ap.error("--dump-outputs writes the images of the sdb200 pipeline; --impl reference times UNet evaluations only")
     if args.impl == "reference":
         run_reference(args)
     else:

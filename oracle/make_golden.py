@@ -43,6 +43,11 @@ def gen(shape, seed, scale=1.0):
     return torch.randn(shape, generator=torch.Generator().manual_seed(seed)) * scale
 
 
+def drawn(kind, shape, seed):
+    """A seeded input stored as its draw (no file over 1 MB): tests/helpers.golden() draws it again, bit for bit."""
+    return {kind: tuple(shape), "seed": seed}
+
+
 @torch.no_grad()
 def unet_goldens():
     cases = []
@@ -63,7 +68,7 @@ def unet_goldens():
             mine = O.unet_forward(sd, x, t, ctx, num_heads=cfg["num_heads"])
             print(f"unet {tag} {xs} t={ts}: ref {dt:.1f}s  eps std {float(eps.std()):.3f} absmax {float(eps.abs().max()):.2f}"
                   f"  oracle rel-L2 {rel(mine, eps):.2e}")
-            cases.append(dict(cfg=tag, x=x, t=t, ctx=ctx, eps=eps, seed=UNET_SEED))
+            cases.append(dict(cfg=tag, x=x, t=t, ctx=drawn("randn", ctx.shape, 200 + i), eps=eps, seed=UNET_SEED))
         del net
     save("unet.pt", cases)
 
@@ -274,7 +279,8 @@ def safety_goldens():
             emb = model(pixel_values=pix).image_embeds
         mine = O.clip_vision_embeds(sd, pix, cfg["num_attention_heads"], cfg["layer_norm_eps"])
         print(f"safety {tag}: embeds std {float(emb.std()):.3f}; oracle rel {rel(mine, emb):.2e}")
-        cases.append(dict(cfg=tag, images=img if tag == "tiny" else None, pixel_values=pix.half() if tag != "tiny" else pix,
+        images = drawn("rand", img.shape, 600) if tag == "tiny" else None
+        cases.append(dict(cfg=tag, images=images, pixel_values=pix.half() if tag != "tiny" else pix,
                           image_embeds=emb, seed=SAFETY_SEED))   # (sdv1: fp16 pixels keep the fixture small; the
         if tag != "tiny":                                          #  embeds below are those OF the rounded pixels)
             with torch.no_grad():
@@ -327,7 +333,9 @@ def fullsize_goldens():
         out["vae"].append(dict(cfg="sdv1", seed=VAE_SEED, latent=lat, z_seed=zseed, img_seed=zseed + 10,
                                dec_sub=_sub(dec), dec_norm=float(dec.double().norm()), dec_mean=float(dec.double().mean()),
                                dec_crop=dec[..., 100:164, 200:264].contiguous(), moments=raw_moments))
-    save("fullsize.pt", out)
+    save("fullsize_unet.pt", out["unet"])
+    for v in out["vae"]:
+        save(f"fullsize_vae_{v['latent']}.pt", v)
 
 
 if __name__ == "__main__":

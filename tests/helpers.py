@@ -20,10 +20,25 @@ CFGS = {"unet": {"tiny": arch.TINY_UNET, "sdv1": arch.SD_V1_UNET},
 _SHAPES = {"unet": arch.unet_param_shapes, "vae": arch.vae_param_shapes, "clip": arch.clip_param_shapes,
            "safety": arch.safety_param_shapes}
 _cache = {}
+_DRAWS = {"randn": torch.randn, "rand": torch.rand}
+
+
+def _redraw(o):
+    if isinstance(o, dict):
+        kind = set(o) - {"seed"}
+        if "seed" in o and len(kind) == 1 and kind <= set(_DRAWS):
+            kind = kind.pop()
+            return _DRAWS[kind](o[kind], generator=torch.Generator().manual_seed(o["seed"]))
+        return {k: _redraw(v) for k, v in o.items()}
+    if isinstance(o, list):
+        return [_redraw(v) for v in o]
+    return o
 
 
 def golden(name):
-    return torch.load(os.path.join(GOLDEN, name), weights_only=True)
+    """A fixture stores a seeded random input as the draw that made it, {"randn" or "rand": shape, "seed": s}
+    (oracle/make_golden.py); it is drawn again here, bit for bit the tensor the reference was given."""
+    return _redraw(torch.load(os.path.join(GOLDEN, name), weights_only=True))
 
 
 def weights(kind, tag, seed):

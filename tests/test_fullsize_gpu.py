@@ -23,7 +23,7 @@ def _sub(t, stride=4, off=1):
 @pytest.mark.parametrize("idx", range(2))
 def test_unet_fullsize_vs_reference(cuda_dev, idx):
     import sdb200
-    case = golden("fullsize.pt")["unet"][idx]
+    case = golden("fullsize_unet.pt")[idx]
     m = sdb200.UNetModel(**CFGS["unet"]["sdv1"]).load_weights(weights("unet", "sdv1", case["seed"]), cuda_dev)
     x = _gen(case["x_shape"], case["x_seed"])
     ctx = _gen((case["x_shape"][0], 77, 768), case["ctx_seed"])
@@ -68,7 +68,7 @@ def test_unet_c3_batch_rows_equal_their_ns2_evaluation(cuda_dev):
 @pytest.mark.parametrize("idx", range(2))
 def test_vae_fullsize_vs_reference(cuda_dev, idx):
     import sdb200
-    case = golden("fullsize.pt")["vae"][idx]
+    case = golden(f"fullsize_vae_{(64, 96)[idx]}.pt")
     lat = case["latent"]
     vae = sdb200.AutoencoderKL(**CFGS["vae"]["sdv1"]).load_weights(weights("vae", "sdv1", case["seed"]), cuda_dev)
     z = _gen((1, 4, lat, lat), case["z_seed"])

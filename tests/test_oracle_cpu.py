@@ -103,18 +103,17 @@ def test_samplers_oracle_50_steps_and_img2img():
 
 
 def test_oracle_matches_reference_fullsize_fixtures():
-    """BASELINE-size fixtures (tests/golden/fullsize.pt, written by the unmodified reference): the oracle reproduces the
+    """BASELINE-size fixtures (tests/golden/fullsize_*.pt, written by the unmodified reference): the oracle reproduces the
     second-weight-seed C1 eps to fp32 round-off (bit-exactly on the host that wrote the fixtures; MKL / oneDNN pick their
     blocking and reduction order from the core count, so another host differs in the last bits: 2.4e-6 on an 8-core
     container) and the 512^2 VAE decode likewise (the 96x96 cases need ~20 GB and half a minute each; make_golden.py
     prints their oracle error when the fixtures are made)."""
     import ldm_oracle as O
-    fs = golden("fullsize.pt")
-    case = fs["unet"][1]
+    case = golden("fullsize_unet.pt")[1]
     g = lambda shape, seed: torch.randn(shape, generator=torch.Generator().manual_seed(seed))
     x, ctx = g(case["x_shape"], case["x_seed"]), g((case["x_shape"][0], 77, 768), case["ctx_seed"])
     eps = O.unet_forward(weights("unet", "sdv1", case["seed"]), x, case["t"], ctx)
     assert torch.equal(eps, case["eps"]) or rel_l2(eps, case["eps"]) < 1e-5
-    v = fs["vae"][0]
+    v = golden("fullsize_vae_64.pt")
     dec = O.vae_decode(weights("vae", "sdv1", v["seed"]), g((1, 4, v["latent"], v["latent"]), v["z_seed"]))
     assert rel_l2(dec[..., 1::4, 1::4], v["dec_sub"]) < 5e-6 and abs(float(dec.double().norm()) / v["dec_norm"] - 1) < 1e-6
