@@ -85,7 +85,6 @@ typedef struct sdb_gemm_desc {
                             (no atomics, no zeroing, bit-reproducible) — the GroupNorm statistics of the tensor being
                             produced, so no separate reduction pass reads it again. T comes from sdb_gemm_plan; the
                             consumer (sdb_groupnorm) folds the T slots */
-  int32_t stats_prezeroed; /* unused (kept for layout compatibility) */
   int32_t b_dynamic;       /* non-zero: b is an activation produced by the preceding kernel (e.g. V^T = W_v . X^T swaps
                               the operand roles), so it must not be prefetched ahead of the programmatic-launch wait */
   int32_t conv_stride;     /* taps = 9 only. 0/1: stride 1. 2: stride-2 conv read straight from the NHWC input through
@@ -163,28 +162,24 @@ int sdb_softmax_rows(const float* x, int32_t rows, int32_t cols, float scale, vo
 int sdb_nchw_to_nhwc(const float* x, int32_t nb, int32_t c, int32_t hw, float* out_f32, void* out_f16,
                      sdb_stream_t stream);
 int sdb_nhwc_to_nchw(const float* x, int32_t nb, int32_t c, int32_t hw, float* out, sdb_stream_t stream);
-/* explicit im2col for the few convs the TMA path does not cover (C_in not a multiple of 64, stride 2,
- * asymmetric pad): out fp16 [nb*ho*wo, kpad], k = (ky*3+kx)*c + ch, zero padded to kpad.
- * pad_lo applies top/left, bottom/right pad is implied by ho/wo (openaimodel.py:149-153; model.py:72-76). */
-int sdb_im2col3x3(const float* x, int32_t nb, int32_t h, int32_t w, int32_t c, int32_t stride, int32_t pad_lo,
-                  int32_t ho, int32_t wo, int32_t kpad, void* out_f16, sdb_stream_t stream);
+/* explicit im2col for the 3x3 convs whose C_in is not a multiple of 64, which the TMA path does not cover (UNet
+ * conv_in, openaimodel.py:519; VAE conv_in, model.py:383,487): stride 1, zero pad 1, NHWC fp32 [nb, h, w, c] ->
+ * fp16 [nb*h*w, kpad], k = (ky*3+kx)*c + ch, zero padded to kpad. */
+int sdb_im2col3x3(const float* x, int32_t nb, int32_t h, int32_t w, int32_t c, int32_t kpad, void* out_f16,
+                  sdb_stream_t stream);
 /* nearest 2x upsample NHWC fp32 -> fp16 (openaimodel.py:116; model.py:54) */
 int sdb_upsample2x(const float* x, int32_t nb, int32_t h, int32_t w, int32_t c, void* out_f16, sdb_stream_t stream);
 /* fp32 -> fp16 cast, optional transpose of [rows, cols] per batch into [cols, ldo] */
 int sdb_cast_f16(const float* x, int64_t n, void* out_f16, sdb_stream_t stream);
 int sdb_transpose_f16(const void* x, int32_t batch, int32_t rows, int32_t cols, int32_t ldx, void* out,
                       int32_t ldo, sdb_stream_t stream);
-/* sinusoidal timestep embedding [cos | sin] (util.py:151-171): t[n] -> fp16 [n, dim] */
-int sdb_timestep_embedding(const float* t, int32_t n, int32_t dim, float max_period, void* out_f16,
-                           sdb_stream_t stream);
-/* fp32 variant of the above, and the small-M fp32-activation linear (time_embed MLP + all emb_layers,
- * openaimodel.py:506-511,217-223): out[m, j] = act(x[m, :] . w[j, :] + bias[j]), w fp16 [n, k], act NONE|SILU */
+/* sinusoidal timestep embedding [cos | sin] (util.py:151-171): t[n] -> fp32 [n, dim]; and the small-M
+ * fp32-activation linear (time_embed MLP + all emb_layers, openaimodel.py:506-511,217-223):
+ * out[m, j] = act(x[m, :] . w[j, :] + bias[j]), w fp16 [n, k], act NONE|SILU */
 int sdb_timestep_embedding_f32(const float* t, int32_t n, int32_t dim, float max_period, float* out,
                                sdb_stream_t stream);
 int sdb_linear_small(const float* x, int32_t m, int32_t k, const void* w_f16, int32_t n, const float* bias,
                      int32_t act, float* out_f32, void* out_f16, sdb_stream_t stream);
-/* y = silu(x) fp32 -> fp16 */
-int sdb_silu_f16(const float* x, int64_t n, void* out_f16, sdb_stream_t stream);
 
 /*
  * One fused sampler update (classifier-free guidance + PLMS / DDIM step), replacing ~25 elementwise
@@ -293,7 +288,6 @@ typedef struct sdb_plan sdb_plan;
 int sdb_plan_begin(sdb_plan** out);
 int sdb_plan_end(sdb_plan* plan);
 int sdb_plan_size(const sdb_plan* plan);                 /* recorded launches (-1: NULL) */
-int sdb_plan_run(sdb_plan* plan, sdb_stream_t stream);    /* eager replay, call by call */
 int sdb_plan_launch(sdb_plan* plan, sdb_stream_t stream); /* graph replay */
 int sdb_plan_destroy(sdb_plan* plan);
 int sdb_fill_f32(float* x, int64_t n, float value, sdb_stream_t stream);

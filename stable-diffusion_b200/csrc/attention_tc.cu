@@ -920,12 +920,7 @@ extern "C" int sdb_attention(const sdb_attn_desc* d, sdb_stream_t stream) {
     if (make_tmap_f16(&tk, d->k, 3, dims, str, box)) return 1;
   }
   // split-state kernel (two threads per query row, row sums from a ones row of V^T): dpad 64 with spare rows
-  static int split_off = -1;
-  if (split_off < 0) {
-    const char* e = getenv("SDB_ATTN_SPLIT");
-    split_off = (e && e[0] == '0') ? 1 : 0;
-  }
-  const bool use_split = d->dpad == 64 && d->d < 64 && d->d % 8 == 0 && !split_off;
+  const bool use_split = d->dpad == 64 && d->d < 64 && d->d % 8 == 0;
   {
     uint64_t dims[3] = {static_cast<uint64_t>(d->nkv), hd, static_cast<uint64_t>(d->batch)};
     uint64_t str[2] = {static_cast<uint64_t>(d->ldvt) * 2, static_cast<uint64_t>(d->vt_batch_stride) * 2};

@@ -51,20 +51,21 @@ __global__ void nhwc_to_nchw_kernel(const float* __restrict__ x, int c, int hw, 
   }
 }
 
-__global__ void im2col3x3_kernel(const float* __restrict__ x, int nb, int h, int w, int c, int stride, int pad_lo,
-                                 int ho, int wo, int kpad, __half* __restrict__ out) {
-  size_t total = static_cast<size_t>(nb) * ho * wo * kpad;
+// 3x3 conv patches, stride 1, zero pad 1: NHWC fp32 -> fp16 [nb*h*w, kpad]
+__global__ void im2col3x3_kernel(const float* __restrict__ x, int nb, int h, int w, int c, int kpad,
+                                 __half* __restrict__ out) {
+  size_t total = static_cast<size_t>(nb) * h * w * kpad;
   GRID_STRIDE(i, total) {
     int k = static_cast<int>(i % kpad);
     size_t row = i / kpad;
     float v = 0.f;
     if (k < 9 * c) {
       int tap = k / c, ch = k - tap * c;
-      int ox = static_cast<int>(row % wo);
-      int oy = static_cast<int>((row / wo) % ho);
-      int n = static_cast<int>(row / (static_cast<size_t>(wo) * ho));
-      int iy = oy * stride + tap / 3 - pad_lo;
-      int ix = ox * stride + tap % 3 - pad_lo;
+      int ox = static_cast<int>(row % w);
+      int oy = static_cast<int>((row / w) % h);
+      int n = static_cast<int>(row / (static_cast<size_t>(w) * h));
+      int iy = oy + tap / 3 - 1;
+      int ix = ox + tap % 3 - 1;
       if (iy >= 0 && iy < h && ix >= 0 && ix < w) v = x[((static_cast<size_t>(n) * h + iy) * w + ix) * c + ch];
     }
     out[i] = __float2half_rn(v);
@@ -92,12 +93,6 @@ __global__ void upsample2x_kernel(const float* __restrict__ x, int nb, int h, in
 __global__ void cast_f16_kernel(const float* __restrict__ x, size_t n, __half* __restrict__ out) {
   GRID_STRIDE(i, n) out[i] = __float2half_rn(x[i]);
 }
-__global__ void silu_f16_kernel(const float* __restrict__ x, size_t n, __half* __restrict__ out) {
-  GRID_STRIDE(i, n) {
-    float v = x[i];
-    out[i] = __float2half_rn(v / (1.0f + __expf(-v)));
-  }
-}
 
 // [batch, rows, ldx] (cols valid) -> [batch, cols, ldo] (rows valid). grid = (rows/32, cols/32, batch)
 __global__ void transpose_f16_kernel(const __half* __restrict__ x, int rows, int cols, int ldx, __half* __restrict__ out,
@@ -113,21 +108,6 @@ __global__ void transpose_f16_kernel(const __half* __restrict__ x, int rows, int
   for (int j = threadIdx.y; j < 32; j += blockDim.y) {
     int c = c0 + j, r = r0 + threadIdx.x;
     if (c < cols && r < rows) out[(static_cast<size_t>(b) * cols + c) * ldo + r] = tile[threadIdx.x][j];
-  }
-}
-
-// util.py:151-171: freqs = exp(-ln(max_period) * i / half); emb = [cos(t f) | sin(t f)]
-__global__ void timestep_embedding_kernel(const float* __restrict__ t, int n, int dim, float max_period,
-                                          __half* __restrict__ out) {
-  int half_dim = dim / 2;
-  size_t total = static_cast<size_t>(n) * half_dim;
-  GRID_STRIDE(i, total) {
-    int j = static_cast<int>(i % half_dim);
-    int r = static_cast<int>(i / half_dim);
-    float freq = expf(-logf(max_period) * static_cast<float>(j) / static_cast<float>(half_dim));
-    float a = t[r] * freq;
-    out[static_cast<size_t>(r) * dim + j] = __float2half_rn(cosf(a));
-    out[static_cast<size_t>(r) * dim + half_dim + j] = __float2half_rn(sinf(a));
   }
 }
 
@@ -298,14 +278,12 @@ extern "C" int sdb_nhwc_to_nchw(const float* x, int32_t nb, int32_t c, int32_t h
   SDB_LAUNCH_CHECK();
   return 0;
 }
-extern "C" int sdb_im2col3x3(const float* x, int32_t nb, int32_t h, int32_t w, int32_t c, int32_t stride,
-                             int32_t pad_lo, int32_t ho, int32_t wo, int32_t kpad, void* out_f16,
+extern "C" int sdb_im2col3x3(const float* x, int32_t nb, int32_t h, int32_t w, int32_t c, int32_t kpad, void* out_f16,
                              sdb_stream_t stream) {
-  SDB_REC(sdb_im2col3x3(x, nb, h, w, c, stride, pad_lo, ho, wo, kpad, out_f16, s_));
+  SDB_REC(sdb_im2col3x3(x, nb, h, w, c, kpad, out_f16, s_));
   SDB_CHECK(x && out_f16 && kpad >= 9 * c && kpad % 64 == 0, "sdb_im2col3x3: bad arguments (kpad=%d c=%d)", kpad, c);
-  size_t total = static_cast<size_t>(nb) * ho * wo * kpad;
-  im2col3x3_kernel<<<grid_for(total), 256, 0, ST>>>(x, nb, h, w, c, stride, pad_lo, ho, wo, kpad,
-                                                    static_cast<__half*>(out_f16));
+  size_t total = static_cast<size_t>(nb) * h * w * kpad;
+  im2col3x3_kernel<<<grid_for(total), 256, 0, ST>>>(x, nb, h, w, c, kpad, static_cast<__half*>(out_f16));
   SDB_LAUNCH_CHECK();
   return 0;
 }
@@ -325,13 +303,6 @@ extern "C" int sdb_cast_f16(const float* x, int64_t n, void* out_f16, sdb_stream
   SDB_LAUNCH_CHECK();
   return 0;
 }
-extern "C" int sdb_silu_f16(const float* x, int64_t n, void* out_f16, sdb_stream_t stream) {
-  SDB_REC(sdb_silu_f16(x, n, out_f16, s_));
-  SDB_CHECK(x && out_f16 && n >= 0, "sdb_silu_f16: bad arguments");
-  silu_f16_kernel<<<grid_for(n), 256, 0, ST>>>(x, static_cast<size_t>(n), static_cast<__half*>(out_f16));
-  SDB_LAUNCH_CHECK();
-  return 0;
-}
 extern "C" int sdb_transpose_f16(const void* x, int32_t batch, int32_t rows, int32_t cols, int32_t ldx, void* out,
                                  int32_t ldo, sdb_stream_t stream) {
   SDB_REC(sdb_transpose_f16(x, batch, rows, cols, ldx, out, ldo, s_));
@@ -339,15 +310,6 @@ extern "C" int sdb_transpose_f16(const void* x, int32_t batch, int32_t rows, int
   dim3 grid((rows + 31) / 32, (cols + 31) / 32, batch), block(32, 8);
   transpose_f16_kernel<<<grid, block, 0, ST>>>(static_cast<const __half*>(x), rows, cols, ldx,
                                                static_cast<__half*>(out), ldo);
-  SDB_LAUNCH_CHECK();
-  return 0;
-}
-extern "C" int sdb_timestep_embedding(const float* t, int32_t n, int32_t dim, float max_period, void* out_f16,
-                                      sdb_stream_t stream) {
-  SDB_REC(sdb_timestep_embedding(t, n, dim, max_period, out_f16, s_));
-  SDB_CHECK(t && out_f16 && dim % 2 == 0, "sdb_timestep_embedding: bad arguments");
-  timestep_embedding_kernel<<<grid_for(static_cast<size_t>(n) * dim / 2), 256, 0, ST>>>(
-      t, n, dim, max_period, static_cast<__half*>(out_f16));
   SDB_LAUNCH_CHECK();
   return 0;
 }
@@ -442,7 +404,7 @@ extern "C" int sdb_embed_tokens(const int64_t* ids, int32_t rows, int32_t n_ctx,
   return 0;
 }
 extern "C" const char* sdb_last_error(void) { return sdb::last_error(); }
-extern "C" int sdb_version(void) { return 100; }
+extern "C" int sdb_version(void) { return 101; }
 extern "C" int sdb_sm_count(void) { return sdb::sm_count(); }
 extern "C" long long sdb_launch_count(void) { return sdb::launch_count(); }
 extern "C" long long sdb_debug_trace(void* buf, int64_t n_words) {

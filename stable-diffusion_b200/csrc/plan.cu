@@ -85,11 +85,6 @@ extern "C" int sdb_plan_end(sdb_plan* p) {
 
 extern "C" int sdb_plan_size(const sdb_plan* p) { return p ? static_cast<int>(p->ops.size()) : -1; }
 
-extern "C" int sdb_plan_run(sdb_plan* p, sdb_stream_t stream) {
-  SDB_CHECK(p && p->closed, "sdb_plan_run: plan not recorded");
-  return run_ops(p, static_cast<cudaStream_t>(stream));
-}
-
 extern "C" int sdb_plan_launch(sdb_plan* p, sdb_stream_t stream) {
   SDB_CHECK(p && p->closed, "sdb_plan_launch: plan not recorded");
   SDB_CHECK(!p->ops.empty(), "sdb_plan_launch: empty plan");

@@ -38,7 +38,6 @@ class GemmDesc(C.Structure):
         ("workspace", C.c_void_p),
         ("workspace_floats", C.c_int64),
         ("stats_out", C.c_void_p),
-        ("stats_prezeroed", C.c_int32),
         ("b_dynamic", C.c_int32),
         ("conv_stride", C.c_int32),
         ("conv_shift", C.c_int32),
@@ -88,14 +87,12 @@ SIGNATURES = {
     "sdb_softmax_rows": ([_P, _I, _I, _F, _P, _P], C.c_int),
     "sdb_nchw_to_nhwc": ([_P, _I, _I, _I, _P, _P, _P], C.c_int),
     "sdb_nhwc_to_nchw": ([_P, _I, _I, _I, _P, _P], C.c_int),
-    "sdb_im2col3x3": ([_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P], C.c_int),
+    "sdb_im2col3x3": ([_P, _I, _I, _I, _I, _I, _P, _P], C.c_int),
     "sdb_upsample2x": ([_P, _I, _I, _I, _I, _P, _P], C.c_int),
     "sdb_cast_f16": ([_P, _L, _P, _P], C.c_int),
     "sdb_transpose_f16": ([_P, _I, _I, _I, _I, _P, _I, _P], C.c_int),
-    "sdb_timestep_embedding": ([_P, _I, _I, _F, _P, _P], C.c_int),
     "sdb_timestep_embedding_f32": ([_P, _I, _I, _F, _P, _P], C.c_int),
     "sdb_linear_small": ([_P, _I, _I, _P, _I, _P, _I, _P, _P, _P], C.c_int),
-    "sdb_silu_f16": ([_P, _L, _P, _P], C.c_int),
     "sdb_sampler_step": ([_P, _P, _P, _I, _F, _I, _P, _P, _P, _P, _F, _F, _F, _F, _L, _P, _P, _P, _P, _P], C.c_int),
     "sdb_vae_sample": ([_P, _P, _I, _I, _F, _P, _P], C.c_int),
     "sdb_to_uint8": ([_P, _L, _P, _P], C.c_int),
@@ -116,7 +113,6 @@ SIGNATURES = {
     "sdb_plan_begin": ([C.POINTER(C.c_void_p)], C.c_int),
     "sdb_plan_end": ([_P], C.c_int),
     "sdb_plan_size": ([_P], C.c_int),
-    "sdb_plan_run": ([_P, _P], C.c_int),
     "sdb_plan_launch": ([_P, _P], C.c_int),
     "sdb_plan_destroy": ([_P], C.c_int),
     "sdb_fill_f32": ([_P, _L, _F, _P], C.c_int),

@@ -13,7 +13,6 @@ import torch
 from . import lib as _l
 from .lib import ACT_GEGLU, ACT_NONE, ACT_QUICK_GELU, ACT_SILU, AttnDesc, GemmDesc  # noqa: F401
 
-LAUNCHES = 0        # op calls made through this module
 _GRAPH_LAUNCHES = 0  # kernels replayed from CUDA graphs (counted at capture time, added per replay)
 PROFILE = None      # when a list: gemm()/attention() append (kind, flops, start_event, end_event)
 RECORD = None       # when a list: gemm() appends (desc, algorithmic_flops, keepalive) so bench.py can replay the launches
@@ -38,11 +37,6 @@ def _ptr(t):
 
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
-def _count(n=1):
-    global LAUNCHES
-    LAUNCHES += n
 
 
 def _chk16(t, name):
@@ -168,7 +162,6 @@ def gemm(a0, b, *, a1=None, a2=None, a3=None, nb=None, h=None, w=None, taps=1, b
     if PROFILE is not None:
         e1.record()
         PROFILE.append(("gemm", 2.0 * M * n * b.shape[1], e0, e1, (M, n, b.shape[1], taps)))
-    _count(2 if plan[3] == 1 else 1)
     if out_f16_lo is not None:
         return out_f16, out_f32, out_f16_lo
     return out_f16, out_f32
@@ -222,14 +215,11 @@ def _tune_gemm(d, M, n, rps, stats_ok, stats_group):
     plan = (C.c_int32 * 5)()
     cands = []
     max_slots = 1
-    import os
-    bns = tuple(int(v) for v in os.environ.get("SDB_TUNE_BN", "64,128,160,256").split(","))
-    cgs = tuple(int(v) for v in os.environ.get("SDB_TUNE_CG", "1,2").split(","))
-    for bn in bns:
+    for bn in (64, 128, 160, 256):
         pad = (n + bn - 1) // bn * bn - n
         if bn > 64 and pad >= bn // 2:
             continue
-        for cg in cgs:
+        for cg in (1, 2):
             for sp, mode in ((1, 0), (2, 2), (4, 2), (2, 1), (3, 1), (4, 1), (6, 1), (8, 1), (12, 1), (16, 1)):
                 if mode == 1 and not d.workspace:
                     continue
@@ -304,7 +294,6 @@ def attention(q, k, vt, *, heads, d, dpad, nq, nkv, scale, causal=False, out=Non
     if PROFILE is not None:
         e1.record()
         PROFILE.append(("attention", 4.0 * B * heads * nq * nkv * d, e0, e1, (B, heads, nq, nkv, d)))
-    _count()
     return out
 
 
@@ -334,7 +323,6 @@ def groupnorm(x0, gamma, beta, *, x1=None, groups=32, eps=1e-5, silu=False, want
                                      eps, 1 if silu else 0, _ptr(out), _ptr(raw), _ptr(out_lo), _ptr(raw_lo), _ptr(ws),
                                      _ptr(cs0[0]) if cs0 else None, _ptr(cs1[0]) if cs1 else None, t0, t1, sg,
                                      _stream()), "sdb_groupnorm")
-    _count(1 if cs0 else 3)
     if want_lo or want_raw_lo:
         return out, raw, out_lo, raw_lo
     return out, raw
@@ -349,7 +337,6 @@ def layernorm(x, gamma, beta, eps=1e-5, want_f32=False):
     out32 = torch.empty_like(x) if want_f32 else None
     _l.check(_l.load().sdb_layernorm(_ptr(x), rows, c, _ptr(gamma), _ptr(beta), eps, _ptr(out), _ptr(out32),
                                      _stream()), "sdb_layernorm")
-    _count()
     return (out, out32) if want_f32 else out
 
 
@@ -359,7 +346,6 @@ def softmax_rows(x, scale):
     rows = x.numel() // cols
     out = torch.empty(x.shape, dtype=torch.float16, device=x.device)
     _l.check(_l.load().sdb_softmax_rows(_ptr(x), rows, cols, scale, _ptr(out), _stream()), "sdb_softmax_rows")
-    _count()
     return out
 
 
@@ -369,7 +355,6 @@ def nchw_to_nhwc(x, want_f32=True, want_f16=False):
     o32 = torch.empty((nb, h, w, c), dtype=torch.float32, device=x.device) if want_f32 else None
     o16 = torch.empty((nb, h, w, c), dtype=torch.float16, device=x.device) if want_f16 else None
     _l.check(_l.load().sdb_nchw_to_nhwc(_ptr(x), nb, c, h * w, _ptr(o32), _ptr(o16), _stream()), "sdb_nchw_to_nhwc")
-    _count()
     return o32, o16
 
 
@@ -379,17 +364,15 @@ def nhwc_to_nchw(x, out=None):
     if out is None:
         out = torch.empty((nb, c, h, w), dtype=torch.float32, device=x.device)
     _l.check(_l.load().sdb_nhwc_to_nchw(_ptr(x), nb, c, h * w, _ptr(out), _stream()), "sdb_nhwc_to_nchw")
-    _count()
     return out
 
 
-def im2col3x3(x, stride, pad_lo, ho, wo, kpad):
+def im2col3x3(x, kpad):
+    """x fp32 NHWC [nb, h, w, c] -> fp16 [nb*h*w, kpad]: the 3x3 / stride-1 / pad-1 patches, K zero-padded to kpad."""
     _chk32(x, "x")
     nb, h, w, c = x.shape
-    out = torch.empty((nb * ho * wo, kpad), dtype=torch.float16, device=x.device)
-    _l.check(_l.load().sdb_im2col3x3(_ptr(x), nb, h, w, c, stride, pad_lo, ho, wo, kpad, _ptr(out), _stream()),
-             "sdb_im2col3x3")
-    _count()
+    out = torch.empty((nb * h * w, kpad), dtype=torch.float16, device=x.device)
+    _l.check(_l.load().sdb_im2col3x3(_ptr(x), nb, h, w, c, kpad, _ptr(out), _stream()), "sdb_im2col3x3")
     return out
 
 
@@ -398,7 +381,6 @@ def upsample2x(x):
     nb, h, w, c = x.shape
     out = torch.empty((nb, 2 * h, 2 * w, c), dtype=torch.float16, device=x.device)
     _l.check(_l.load().sdb_upsample2x(_ptr(x), nb, h, w, c, _ptr(out), _stream()), "sdb_upsample2x")
-    _count()
     return out
 
 
@@ -406,15 +388,6 @@ def cast_f16(x):
     _chk32(x, "x")
     out = torch.empty(x.shape, dtype=torch.float16, device=x.device)
     _l.check(_l.load().sdb_cast_f16(_ptr(x), x.numel(), _ptr(out), _stream()), "sdb_cast_f16")
-    _count()
-    return out
-
-
-def silu_f16(x):
-    _chk32(x, "x")
-    out = torch.empty(x.shape, dtype=torch.float16, device=x.device)
-    _l.check(_l.load().sdb_silu_f16(_ptr(x), x.numel(), _ptr(out), _stream()), "sdb_silu_f16")
-    _count()
     return out
 
 
@@ -429,16 +402,6 @@ def transpose_f16(x, ldo=None, out=None):
     assert out.shape == (B, cols, ldo) and out.is_contiguous()
     _l.check(_l.load().sdb_transpose_f16(_ptr(x), B, rows, cols, cols, _ptr(out), ldo, _stream()),
              "sdb_transpose_f16")
-    _count()
-    return out
-
-
-def timestep_embedding(t, dim, max_period=10000.0):
-    _chk32(t, "t")
-    out = torch.empty((t.numel(), dim), dtype=torch.float16, device=t.device)
-    _l.check(_l.load().sdb_timestep_embedding(_ptr(t), t.numel(), dim, max_period, _ptr(out), _stream()),
-             "sdb_timestep_embedding")
-    _count()
     return out
 
 
@@ -447,7 +410,6 @@ def timestep_embedding_f32(t, dim, max_period=10000.0):
     out = torch.empty((t.numel(), dim), dtype=torch.float32, device=t.device)
     _l.check(_l.load().sdb_timestep_embedding_f32(_ptr(t), t.numel(), dim, max_period, _ptr(out), _stream()),
              "sdb_timestep_embedding_f32")
-    _count()
     return out
 
 
@@ -461,7 +423,6 @@ def linear_small(x, w, bias=None, act=ACT_NONE, want_f16=False):
     out16 = torch.empty((m, n), dtype=torch.float16, device=x.device) if want_f16 else None
     _l.check(_l.load().sdb_linear_small(_ptr(x), m, k, _ptr(w), n, _ptr(bias), act, _ptr(out), _ptr(out16),
                                         _stream()), "sdb_linear_small")
-    _count()
     return (out, out16) if want_f16 else out
 
 
@@ -486,7 +447,6 @@ def sampler_step(x, eps2, *, guided, scale, order, hist, noise, a_t, a_prev, sig
                                         _ptr(h[1]), _ptr(h[2]), _ptr(noise), a_t, a_prev, sigma_t,
                                         sqrt_one_minus_a_t, n, _ptr(x_prev), xp2, _ptr(pred_x0), _ptr(e_out),
                                         _stream()), "sdb_sampler_step")
-    _count()
     return x_prev, pred_x0, e_out
 
 
@@ -504,7 +464,6 @@ def dpm_solver_step(x, eps2, *, guided, scale, sigma_s, alpha_s, order, m_prev, 
     _l.check(_l.load().sdb_dpm_solver_step(_ptr(x), _ptr(eps2), _ptr(eps_cond), 1 if guided else 0, scale, sigma_s, alpha_s, order,
                                            _ptr(m_prev), c_x, c_m, inv_r0, n, _ptr(m_out), _ptr(x_out), xo2,
                                            _stream()), "sdb_dpm_solver_step")
-    _count()
     return x_out, m_out
 
 
@@ -519,7 +478,6 @@ def mask_blend(img_orig, mask, img, b, dup=False):
     i2 = C.c_void_p(img.data_ptr() + 4 * img_orig.numel()) if dup else None
     _l.check(_l.load().sdb_mask_blend(_ptr(img_orig), _ptr(mask), mask.shape[1], nb, c, hw, _ptr(img), i2, _stream()),
              "sdb_mask_blend")
-    _count()
     return img
 
 
@@ -528,7 +486,6 @@ def axpby2(x, y, a, b):
     _chk32(y, "y")
     out = torch.empty_like(x)
     _l.check(_l.load().sdb_axpby2(_ptr(x), _ptr(y), a, b, x.numel(), _ptr(out), _stream()), "sdb_axpby2")
-    _count()
     return out
 
 
@@ -537,7 +494,6 @@ def vae_sample(moments, noise, nb, hw, scale_factor):
     z = torch.empty((nb, 4, hw), dtype=torch.float32, device=moments.device)
     _l.check(_l.load().sdb_vae_sample(_ptr(moments), _ptr(noise), nb, hw, scale_factor, _ptr(z), _stream()),
              "sdb_vae_sample")
-    _count()
     return z
 
 
@@ -545,7 +501,6 @@ def to_uint8(x):
     _chk32(x, "x")
     out = torch.empty(x.shape, dtype=torch.uint8, device=x.device)
     _l.check(_l.load().sdb_to_uint8(_ptr(x), x.numel(), _ptr(out), _stream()), "sdb_to_uint8")
-    _count()
     return out
 
 
@@ -557,7 +512,6 @@ def axpby(x, a, b=0.0, out=None):
         _chk32(out, "out")
         assert out.numel() == x.numel()
     _l.check(_l.load().sdb_axpby(_ptr(x), a, b, x.numel(), _ptr(out), _stream()), "sdb_axpby")
-    _count()
     return out
 
 
@@ -570,7 +524,6 @@ def pointwise_small(x, w, b=None, alpha=1.0):
     out = torch.empty(tuple(x.shape[:-1]) + (cout,), dtype=torch.float32, device=x.device)
     _l.check(_l.load().sdb_pointwise_small(_ptr(x), x.numel() // cin, cin, cout, _ptr(w), _ptr(b), alpha, _ptr(out),
                                            _stream()), "sdb_pointwise_small")
-    _count()
     return out
 
 
@@ -582,5 +535,4 @@ def embed_tokens(ids, tok, pos):
     out = torch.empty((B * n, dim), dtype=torch.float32, device=ids.device)
     _l.check(_l.load().sdb_embed_tokens(_ptr(ids), B * n, n, dim, tok.shape[0], _ptr(tok), _ptr(pos), _ptr(out),
                                         _stream()), "sdb_embed_tokens")
-    _count()
     return out

@@ -11,7 +11,6 @@ decision (sdb_safety_scores). State-dict keys are diffusers' (`vision_model.visi
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 
 import numpy as np
@@ -21,16 +20,8 @@ import torch.nn as nn
 from . import lib as _l
 from . import ops
 from .arch import CLIP_IMAGE_MEAN, CLIP_IMAGE_STD, SD_V1_SAFETY, safety_param_shapes
-from .ops import ACT_QUICK_GELU
+from .ops import ACT_QUICK_GELU, _ptr, _stream
 from .util import adopt_state_dict
-
-
-def _ptr(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
 def _bicubic(x):

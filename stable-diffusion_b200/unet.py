@@ -74,11 +74,10 @@ def _pack_geglu(w, b):  # [8C, C]: rows [0,4C) value, [4C,8C) gate -> per accumu
 
 
 class UNetModel(nn.Module):
-    # "fp16x3": the 1x1 convs that act on the raw residual stream (ResBlock skip_connection, SpatialTransformer
-    # proj_in / proj_out) and the final 320->4 conv run with hi/lo-split fp16 operands (three tensor-core passes,
-    # ~fp32 operand precision); everything else single-pass fp16. These few layers (5% of the FLOPs) carry ~60% of the
-    # fp16 operand-rounding error of eps (DESIGN.md, numerics). "fp16": single pass everywhere (eps rel-L2 ~1.2e-3).
-    PRECISION = "fp16x3"
+    # The 1x1 convs that act on the raw residual stream (ResBlock skip_connection, SpatialTransformer proj_in /
+    # proj_out) and the final 320->4 conv run with hi/lo-split fp16 operands (three tensor-core passes, ~fp32 operand
+    # precision); everything else is single-pass fp16. These few layers (5% of the FLOPs) carry ~60% of the fp16
+    # operand-rounding error of eps (DESIGN.md, numerics).
 
     def __init__(self, image_size, in_channels, model_channels, out_channels, num_res_blocks, attention_resolutions,
                  dropout=0, channel_mult=(1, 2, 4, 8), conv_resample=True, dims=2, num_classes=None,
@@ -114,7 +113,6 @@ class UNetModel(nn.Module):
         self.dtype = torch.float32
         self.plan = unet_plan(self.cfg)
         self.shapes = unet_param_shapes(self.cfg)
-        self.precision = self.PRECISION
         # channels per fused GroupNorm-statistics entry: every channel count of the UNet (and of its skip concats) is a
         # multiple of model_channels, so the 32 groups always tile into entries of model_channels / 32 channels
         self._sg = model_channels // 32 if model_channels % 32 == 0 else 1
@@ -161,9 +159,6 @@ class UNetModel(nn.Module):
         W = {"device": device}
         f32 = lambda k: sd[k].contiguous()
         f16 = lambda k: sd[k].half().contiguous()
-        x3 = self.precision == "fp16x3"
-        W["x3"] = x3
-        one = (lambda w: _pack_hilo_1x1(w)) if x3 else (lambda w: w.half().contiguous())
         heads = self.num_heads
         mc = self.model_channels
         W["te0_w"], W["te0_b"] = f16("time_embed.0.weight"), f32("time_embed.0.bias")
@@ -179,7 +174,7 @@ class UNetModel(nn.Module):
             r["gn2"] = (f32(pre + ".out_layers.0.weight"), f32(pre + ".out_layers.0.bias"))
             r["w2"], r["b2"] = _pack_conv3(sd[pre + ".out_layers.3.weight"]), f32(pre + ".out_layers.3.bias")
             if a["cin"] != a["cout"]:
-                r["ws"] = one(sd[pre + ".skip_connection.weight"].reshape(a["cout"], a["cin"]))
+                r["ws"] = _pack_hilo_1x1(sd[pre + ".skip_connection.weight"].reshape(a["cout"], a["cin"]))
                 r["bs"] = f32(pre + ".skip_connection.bias")
             emb_w.append(sd[pre + ".emb_layers.1.weight"].half())
             emb_b.append(sd[pre + ".emb_layers.1.bias"])
@@ -193,8 +188,8 @@ class UNetModel(nn.Module):
             tb = pre + ".transformer_blocks.0"
             s = {"ch": ch, "d": d, "dpad": dp, "heads": heads}
             s["gn"] = (f32(pre + ".norm.weight"), f32(pre + ".norm.bias"))
-            s["w_in"], s["b_in"] = one(sd[pre + ".proj_in.weight"].reshape(ch, ch)), f32(pre + ".proj_in.bias")
-            s["w_out"], s["b_out"] = one(sd[pre + ".proj_out.weight"].reshape(ch, ch)), f32(pre + ".proj_out.bias")
+            s["w_in"], s["b_in"] = _pack_hilo_1x1(sd[pre + ".proj_in.weight"].reshape(ch, ch)), f32(pre + ".proj_in.bias")
+            s["w_out"], s["b_out"] = _pack_hilo_1x1(sd[pre + ".proj_out.weight"].reshape(ch, ch)), f32(pre + ".proj_out.bias")
             for i in (1, 2, 3):
                 s[f"ln{i}"] = (f32(f"{tb}.norm{i}.weight"), f32(f"{tb}.norm{i}.bias"))
             s["w_qk1"] = torch.cat([_pack_heads(sd[tb + ".attn1.to_q.weight"], heads, d, dp),
@@ -229,7 +224,7 @@ class UNetModel(nn.Module):
         W["middle"] = pack_layers(self.plan["middle"])
         W["output"] = [pack_layers(l) for l in self.plan["output"]]
         W["gn_out"] = (f32("out.0.weight"), f32("out.0.bias"))
-        W["w_out"] = _pack_hilo_conv3(sd["out.2.weight"]) if x3 else _pack_conv3(sd["out.2.weight"])
+        W["w_out"] = _pack_hilo_conv3(sd["out.2.weight"])
         W["b_out"] = f32("out.2.bias")
         W["emb_w"] = torch.cat(emb_w, 0).contiguous()
         W["emb_b"] = torch.cat(emb_b, 0).float().contiguous()
@@ -253,19 +248,16 @@ class UNetModel(nn.Module):
         """ResBlock._forward (openaimodel.py:255-275); `skip` is the UNet skip tensor concatenated along C.
         emit_f16: the last GEMM also writes an fp16 copy of the block output (operand of a following stride-2 conv)."""
         nb, H, Wd, _ = h.shape
-        x3 = self.W["x3"] and "ws" in r
-        if x3:
+        if "ws" in r:
             hn, raw, _, raw_lo = ops.groupnorm(h, *r["gn1"], x1=skip, eps=1e-5, silu=True, want_raw_lo=True)
         else:
-            hn, raw = ops.groupnorm(h, *r["gn1"], x1=skip, eps=1e-5, silu=True, want_raw="ws" in r)
+            hn, _ = ops.groupnorm(h, *r["gn1"], x1=skip, eps=1e-5, silu=True)
         fv = film[:, r["film_off"]: r["film_off"] + r["cout"]]
         _, h1 = ops.gemm(hn, r["w1"], taps=9, bias=r["b1"], film=fv, want_f32=True, splits=-1, want_stats=True, stats_group=self._sg)
         h1 = h1.view(nb, H, Wd, r["cout"])
         hn2, _ = ops.groupnorm(h1, *r["gn2"], eps=1e-5, silu=True)
-        if x3:    # skip 1x1 conv on the raw stream: [x_hi | x_lo | x_hi] . [W_hi | W_hi | W_lo]
+        if "ws" in r:    # skip 1x1 conv on the raw stream: [x_hi | x_lo | x_hi] . [W_hi | W_hi | W_lo]
             _, res = ops.gemm(raw, r["ws"], a1=raw_lo, a2=raw, bias=r["bs"], want_f32=True, splits=-1)
-        elif "ws" in r:
-            _, res = ops.gemm(raw, r["ws"], bias=r["bs"], want_f32=True, splits=-1)
         else:
             assert skip is None
             res = h.view(-1, r["cout"])
@@ -283,13 +275,8 @@ class UNetModel(nn.Module):
         heads, d, dp = s["heads"], s["d"], s["dpad"]
         hd = heads * dp
         scale = d ** -0.5
-        x3 = self.W["x3"]
-        if x3:
-            xn, _, xn_lo, _ = ops.groupnorm(x, *s["gn"], eps=1e-6, silu=False, want_lo=True)
-            _, t0 = ops.gemm(xn, s["w_in"], a1=xn_lo, a2=xn, bias=s["b_in"], want_f32=True, splits=-1)
-        else:
-            xn, _ = ops.groupnorm(x, *s["gn"], eps=1e-6, silu=False)
-            _, t0 = ops.gemm(xn, s["w_in"], bias=s["b_in"], want_f32=True, splits=-1)      # tokens [M, ch] fp32
+        xn, _, xn_lo, _ = ops.groupnorm(x, *s["gn"], eps=1e-6, silu=False, want_lo=True)
+        _, t0 = ops.gemm(xn, s["w_in"], a1=xn_lo, a2=xn, bias=s["b_in"], want_f32=True, splits=-1)   # tokens [M, ch] fp32
         # --- self attention
         y = ops.layernorm(t0, *s["ln1"])
         qk, _ = ops.gemm(y, s["w_qk1"], want_f16=True)                                     # [M, 2*hd]
@@ -313,14 +300,9 @@ class UNetModel(nn.Module):
         y = ops.layernorm(t2, *s["ln3"])
         g, _ = ops.gemm(y, s["w_ff1"], bias=s["b_ff1"], act=ACT_GEGLU, want_f16=True,
                         block_n=_geglu_tile(s["w_ff1"].shape[0] // 2))
-        if x3:
-            t3, _, t3_lo = ops.gemm(g, s["w_ff2"], bias=s["b_ff2"], residual=t2, want_lo=True, splits=-1)
-            o16, out = ops.gemm(t3, s["w_out"], a1=t3_lo, a2=t3, bias=s["b_out"], residual=x.view(-1, ch), want_f32=True,
-                                want_f16=emit_f16, splits=-1, rows_per_sample=ntok, want_stats=True, stats_group=self._sg)
-        else:
-            t3, _ = ops.gemm(g, s["w_ff2"], bias=s["b_ff2"], residual=t2, want_f16=True, splits=-1)
-            o16, out = ops.gemm(t3, s["w_out"], bias=s["b_out"], residual=x.view(-1, ch), want_f32=True,
-                                want_f16=emit_f16, splits=-1, rows_per_sample=ntok, want_stats=True, stats_group=self._sg)
+        t3, _, t3_lo = ops.gemm(g, s["w_ff2"], bias=s["b_ff2"], residual=t2, want_lo=True, splits=-1)
+        o16, out = ops.gemm(t3, s["w_out"], a1=t3_lo, a2=t3, bias=s["b_out"], residual=x.view(-1, ch), want_f32=True,
+                            want_f16=emit_f16, splits=-1, rows_per_sample=ntok, want_stats=True, stats_group=self._sg)
         out = out.view(nb, H, Wd, ch)
         if emit_f16:
             out._sdb_f16 = o16.view(nb, H, Wd, ch)
@@ -392,7 +374,7 @@ class UNetModel(nn.Module):
                 h = o.view(nb, 2 * H, 2 * Wd, c)
             elif kind == "conv_in":
                 nb, H, Wd, c = h.shape
-                col = ops.im2col3x3(h, 1, 1, H, Wd, 64)
+                col = ops.im2col3x3(h, 64)
                 _, o = ops.gemm(col, p["w"], bias=p["b"], want_f32=True, rows_per_sample=H * Wd, want_stats=True, stats_group=self._sg)
                 h = o.view(nb, H, Wd, p["cout"])
         return h
@@ -439,12 +421,8 @@ class UNetModel(nn.Module):
         h = self._run_layers(W["middle"], h, None, film, kvs, st_idx)
         for layers in W["output"]:
             h = self._run_layers(layers, h, hs.pop(), film, kvs, st_idx)
-        if W["x3"]:
-            hn, _, hn_lo, _ = ops.groupnorm(h, *W["gn_out"], eps=1e-5, silu=True, want_lo=True)
-            _, o = ops.gemm(hn, W["w_out"], a1=hn_lo, a2=hn, taps=9, bias=W["b_out"], want_f32=True)
-        else:
-            hn, _ = ops.groupnorm(h, *W["gn_out"], eps=1e-5, silu=True)
-            _, o = ops.gemm(hn, W["w_out"], taps=9, bias=W["b_out"], want_f32=True)
+        hn, _, hn_lo, _ = ops.groupnorm(h, *W["gn_out"], eps=1e-5, silu=True, want_lo=True)
+        _, o = ops.gemm(hn, W["w_out"], a1=hn_lo, a2=hn, taps=9, bias=W["b_out"], want_f32=True)
         return ops.nhwc_to_nchw(o.view(nb, H, Wd, self.out_channels))
 
     def _graph_for(self, shape, kvs):

@@ -153,7 +153,7 @@ class AutoencoderKL(nn.Module):
         """3x3 conv pad 1: TMA implicit GEMM when C_in % 64 == 0, else explicit im2col (3/4-channel inputs)."""
         if c["col"]:
             nb, H, Wd, _ = x32.shape
-            col = ops.im2col3x3(x32, 1, 1, H, Wd, c["w"].shape[1])
+            col = ops.im2col3x3(x32, c["w"].shape[1])
             _, o = ops.gemm(col, c["w"], bias=c["b"], want_f32=True, rows_per_sample=H * Wd, want_stats=True,
                             stats_group=_sg(c["cout"]), **epi)
             return o.view(nb, H, Wd, c["cout"])

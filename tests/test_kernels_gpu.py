@@ -352,29 +352,23 @@ def test_elementwise(S, cuda_dev):
     o32, o16 = S.ops.nchw_to_nhwc(x, want_f16=True)
     assert torch.equal(o32, x.permute(0, 2, 3, 1).contiguous())
     assert torch.equal(S.ops.nhwc_to_nchw(o32), x)
-    # im2col: stride 2 pad 1 and asymmetric (pad_lo 0)
+    # im2col: 3x3, stride 1, pad 1
     xi = torch.randn(2, 9, 9, 4, generator=g).to(cuda_dev)
-    for stride, pad_lo, ho in [(1, 1, 9), (2, 1, 5), (2, 0, 4)]:
-        col = S.ops.im2col3x3(xi, stride, pad_lo, ho, ho, 64)
-        xp = xi.permute(0, 3, 1, 2)
-        if pad_lo == 0:
-            xp = F.pad(xp, (0, 1, 0, 1))
-            un = F.unfold(xp, 3, stride=stride)
-        else:
-            un = F.unfold(xp, 3, stride=stride, padding=1)
-        # unfold: [nb, c*9, L] with index c*9 + tap -> ours tap*c + ch
-        un = un.reshape(2, 4, 9, -1).permute(0, 3, 2, 1).reshape(-1, 36)
-        assert torch.allclose(col[:, :36].float(), un, atol=2e-3)
-        assert float(col[:, 36:].abs().max()) == 0.0
+    col = S.ops.im2col3x3(xi, 64)
+    un = F.unfold(xi.permute(0, 3, 1, 2), 3, padding=1)
+    # unfold: [nb, c*9, L] with index c*9 + tap -> ours tap*c + ch
+    un = un.reshape(2, 4, 9, -1).permute(0, 3, 2, 1).reshape(-1, 36)
+    assert torch.allclose(col[:, :36].float(), un, atol=2e-3)
+    assert float(col[:, 36:].abs().max()) == 0.0
     up = S.ops.upsample2x(o32)
     assert torch.allclose(up.float(), F.interpolate(x, scale_factor=2, mode="nearest").permute(0, 2, 3, 1), atol=2e-3)
     t = torch.tensor([981.0, 1.0, 500.5], device=cuda_dev)
-    te = S.ops.timestep_embedding(t, 320)
+    te = S.ops.timestep_embedding_f32(t, 320)
     half = 160
     freqs = torch.exp(-math.log(10000) * torch.arange(half, dtype=torch.float32, device=cuda_dev) / half)
     args = t[:, None] * freqs[None]
     ref = torch.cat([torch.cos(args), torch.sin(args)], -1)
-    assert float((te.float() - ref).abs().max()) < 2e-3
+    assert te.dtype == torch.float32 and float((te - ref).abs().max()) < 2e-3
     tr = S.ops.transpose_f16(o16.reshape(2, 64, 8))
     assert tr.shape == (2, 8, 64) and torch.equal(tr, o16.reshape(2, 64, 8).transpose(1, 2))
 
